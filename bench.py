@@ -14,7 +14,11 @@ reads its predecessor's output; the out projection reads the first M x 3072 elem
 the attention output.  Attention itself and the AdaLN modulation GEMVs are outside the hot path and not run.
 An image is 4 steps.  value = images/s of this stack, whole job over all ranks (replicas, no collective in the timed path).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--precision nvfp4|int4] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--precision nvfp4|int4] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned (the hidden states after the 57 blocks, [4352, 3072]) as
+DIR/hidden_states.npy in float32 (53 MB).  Inputs and weights come from fixed seeds, so two builds run with the same arguments
+can be compared output for output.
 
 One JSON line on stdout (driver contract + roofline, cpu_baseline, e2e, clocks, gpu_launches, reference_gpu, cublas_bf16).
 """
@@ -636,6 +640,15 @@ def _emit(line: dict) -> None:
         sys.stdout.flush()
 
 
+def dump_outputs(path: str, arrays: dict) -> None:
+    """--dump-outputs: every array as DIR/<name>.npy, float32"""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.float().cpu().numpy())
+
+
 def load_peaks():
     """roofline denominators: tensor-pipe peaks measured on a B200 by tools/ubench/mma_peak.cu (committed: profiles/r02_mma_peaks.json)
     and the driver's MEASURED_PEAKS.json (HBM, cuBLAS bf16)."""
@@ -664,7 +677,10 @@ def main() -> int:
     ap.add_argument("--no-full", action="store_true", help="skip the whole-transformer-step figure (attention + AdaLN modulation on top of the linear stack)")
     ap.add_argument("--no-graph", action="store_true", help="time eager launches instead of a captured CUDA graph")
     ap.add_argument("--skip-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's hidden states to DIR/hidden_states.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference_arm(args)
@@ -712,6 +728,8 @@ def main() -> int:
     stepper = graph if graph is not None else Eager()
     with ClockSampler(local) as clocks:
         ms = time_replays(torch, stepper, args.steps, barrier)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"hidden_states": runner.result})
     ms_per_step = replica.max_over_ranks(ms, device) / args.steps
     images_per_s = world * (1.0 / STEPS_PER_IMAGE) / (ms_per_step * 1e-3)
     f_main, f_lr = step_flops()

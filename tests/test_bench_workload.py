@@ -1,10 +1,14 @@
-"""CPU: the bench's synthetic workload is the one BASELINE.json / SURVEY.md section 8(d) name -- FLUX.1-schnell 1024x1024,
+"""The bench's synthetic workload is the one BASELINE.json / SURVEY.md section 8(d) name -- FLUX.1-schnell 1024x1024,
 dim 3072, 24 heads, mlp 12288, rank 32, 19 joint + 38 single blocks, 4096 image + 256 text tokens -- and its FLOP
-bookkeeping matches SURVEY's figure (57 blocks x 113.25 M 4-bit params x 2 x tokens = 56.2 TFLOP per step)."""
+bookkeeping matches SURVEY's figure (57 blocks x 113.25 M 4-bit params x 2 x tokens = 56.2 TFLOP per step); its command line
+(CPU) and, on the GPU, the outputs it dumps for comparing two builds."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 import bench
 
@@ -43,6 +47,25 @@ def test_reference_arm_prints_one_json_line():
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["value"] == d["value"] == d["e2e"]["value"]
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
     assert d["metric"].startswith("FLUX.1-schnell") and "workload" in d["config"]
+
+
+def test_steps_must_be_positive():
+    pr = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"], capture_output=True, text=True, timeout=120)
+    assert pr.returncode == 2 and "--steps" in pr.stderr and not pr.stdout.strip()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_writes_the_last_timed_step(tmp_path):
+    """`--dump-outputs DIR`: the hidden states the timed path returned, float32, within 64 MB; `--steps` is the number of timed steps."""
+    pr = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "0", "--no-secondary", "--no-legs", "--no-full",
+                         "--skip-cpu", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900)
+    assert pr.returncode == 0, pr.stderr[-2000:]
+    lines = [l for l in pr.stdout.splitlines() if l.strip()]
+    assert len(lines) == 1 and json.loads(lines[0])["steps"] == 2
+    assert [p.name for p in tmp_path.iterdir()] == ["hidden_states.npy"] and (tmp_path / "hidden_states.npy").stat().st_size <= 64 << 20
+    y = np.load(tmp_path / "hidden_states.npy")
+    assert y.dtype == np.float32 and y.shape == (bench.IMG_TOKENS + bench.TXT_TOKENS, bench.DIM)
+    assert np.isfinite(y).all() and y.std() > 0
 
 
 def test_host_threads_respects_the_cgroup_quota(monkeypatch):

@@ -1,6 +1,7 @@
 """GPU parity of the AWQ W4A16 GEMV (SURVEY section 8f row N2): against the oracle (oracle/awq.py, bit-exact with the reference's kernel
-on its golden vectors: tests/test_ref_gpu_golden.py), against the committed reference-on-B200 outputs themselves, and -- when the
-reference library is present -- against the reference kernel live at the FLUX AdaLN sizes."""
+on its golden vectors: tests/test_ref_gpu_golden.py), against the committed reference-on-B200 outputs themselves, at the FLUX AdaLN
+sizes against the reference kernel's recorded outputs (tests/golden/make_ref_parity_golden.py), and -- when the seam library is
+built -- through the reference's own host entry point."""
 import os
 
 import numpy as np
@@ -56,25 +57,34 @@ def test_gemv_awq_vs_oracle_and_layer(m, hT):
     _close(y, want, f"oracle {hT} m={m}")
 
 
-def test_gemv_awq_flux_adaln_size_vs_reference_kernel_live():
-    """FLUX AdaLN: 3072 -> 18432 (6 x dim), batch 1: our kernel vs the reference's, same checkpoint bytes, same GPU"""
-    from oracle import refgpu as R
-
-    if not R.available("ref"):
-        pytest.skip("oracle/_ref/libnunchaku_ref.so not built")
-    from nunchaku_b200.ops.gemv import awq_gemv_w4a16_cuda
-
+def adaln_case():
+    """-> (qweight, [(dtype, scales, zeros, x)]) in the order they are drawn"""
     g = torch.Generator(device="cuda").manual_seed(5)
     OC, IC = 18432, 3072
     qw = torch.randint(-2 ** 31, 2 ** 31 - 1, (OC // 4, IC // 2), generator=g, device="cuda", dtype=torch.int64).to(torch.int32)
+    per = []
     for hT in (torch.bfloat16, torch.float16):
         sc = (torch.rand(IC // 64, OC, generator=g, device="cuda") * 0.02 + 0.005).to(hT)
         ze = (-(torch.rand(IC // 64, OC, generator=g, device="cuda") * 0.1 + 0.03)).to(hT)
         x = torch.randn(1, IC, generator=g, device="cuda").to(hT)
+        per.append((hT, sc, ze, x))
+    return qw, per
+
+
+def test_gemv_awq_flux_adaln_size_vs_reference_kernel_live():
+    """FLUX AdaLN: 3072 -> 18432 (6 x dim), batch 1: our kernel vs what the reference's kernel computed on a B200 from the same
+    checkpoint bytes"""
+    from gpu_util import ref_golden, sample
+    from nunchaku_b200.ops.gemv import awq_gemv_w4a16_cuda
+
+    qw, per = adaln_case()
+    OC, IC = qw.shape[0] * 4, qw.shape[1] * 2
+    gold = ref_golden("awq_adaln", qw, *[t for _, sc, ze, x in per for t in (sc, ze, x)])
+    for hT, sc, ze, x in per:
         y = awq_gemv_w4a16_cuda(x, qw, sc, ze, 1, OC, IC, 64)
-        want = R.gemv_awq(x, qw, sc, ze, 1, OC, IC, 64)
         torch.cuda.synchronize()
-        _close(y, want, f"live {hT}")
+        want = gold[str(hT).split(".")[-1]]
+        _close(sample(y, want.numel()), want, f"live {hT}")
 
 
 def test_gemv_awq_through_the_cpp_seam_and_the_pybind_surface():
